@@ -2,6 +2,7 @@
 """Benchmark of the NLP oracle hot path: oracle evals/s for the set (f, grad f, g, J, Hess L).
 
     python bench.py --gpus N --steps K --warmup W [--workload all|c1|c2|c3|c4|c5] [--impl reference]
+                    [--dump-outputs DIR]
 
 Headline workload (every N): BASELINE config 3, the sparse logistic-type regression m = 2 M, n = 4096 -
 the configuration the metric is quoted on "at 1/2/4/8 B200": one GPU evaluates it whole, N > 1 GPUs
@@ -11,7 +12,11 @@ as sub-results: c2 (dense eigen-QCQP, one GPU), c5 (10 M-node DAG + 50 M-nnz Jac
 (4096-start multi-start batch, starts split over the N ranks, no collective).
 
 One STEP = `evals_per_step` evaluations of all five quantities, every cache invalidated before each
-evaluation; `evals_per_step` is chosen so that the K timed steps last about a second.
+evaluation; `evals_per_step` is chosen so that one step lasts about 50 ms, and K timed steps are run.
+
+--dump-outputs DIR writes what the device-resident path computed in its last timed step (the five
+outputs of every workload run, DIR/<workload>_<output>.npy, float64), so that two builds can be
+compared output for output: the inputs are seeded and the same for the same arguments.
 
   value     device-side throughput: (x, lambda, sigma) resident in HBM, CUDA events on the oracle's own
             stream, max over ranks.  N > 1: the exchange of shared entries is inside the timed region.
@@ -46,9 +51,10 @@ METRIC = "oracle evals/s (f, grad f, g, J, Hess L)"
 # profiles/r01_cublas_dgemm.txt) reached 35.4 TFLOP/s, 27.3 at the C4 shape [512x512]x[512x4096].
 FP64_TENSOR_PEAK = 35.4
 FP64_TENSOR_PEAK_SRC = "measured: cuBLAS DGEMM 4096^3 on this pool (profiles/r01_cublas_dgemm.txt); nominal 40"
-TARGET_TIMED_S = 1.0          # the K timed steps should last about this long (device leg)
+TARGET_STEP_S = 0.05          # one timed step of the device leg should last about this long
 HBM_SPEC_GBS = 8000.0            # the nominal figure north_star quotes next to the measured copy bandwidth
-TARGET_E2E_S = 0.6
+TARGET_E2E_STEP_S = 0.03      # one timed step of the e2e leg
+DUMP_MAX_ENTRIES = 1 << 18    # --dump-outputs: entries kept per output (5 workloads x 5 outputs x 2 MB < 64 MB)
 
 
 # ------------------------------------------------------------------ workloads
@@ -328,7 +334,7 @@ def timed_device(run, grp, steps, warmup, clock_index):
     ranks), evals_per_step, clocks)."""
     run(3)
     probe = max(float(grp.max([run(8) / 8.0])[0]), 1e-4)                 # ms per evaluation
-    E = max(1, int(math.ceil(TARGET_TIMED_S * 1e3 / (steps * probe))))
+    E = max(1, int(math.ceil(TARGET_STEP_S * 1e3 / probe)))
     nwarm = max(warmup, 3) * E
     run(nwarm if nwarm * probe < 2000 else max(3, int(2000 / probe)))
     grp.barrier()
@@ -347,7 +353,7 @@ def timed_e2e(five, grp, steps):
     t0 = time.perf_counter()
     five(2), five(3)
     probe = float(grp.max([(time.perf_counter() - t0) / 2.0])[0])
-    E = max(1, int(math.ceil(TARGET_E2E_S / (steps * max(probe, 1e-6)))))
+    E = max(1, int(math.ceil(TARGET_E2E_STEP_S / max(probe, 1e-6))))
     grp.barrier()
     t0 = time.perf_counter()
     for i in range(steps * E):
@@ -365,6 +371,18 @@ def parity_excess(got, want, rtol=1e-10, atol_rel=1e-12):
         return 0.0
     scale = float(np.max(np.abs(b))) if b.size else 0.0
     return float(np.max(np.abs(a - b) / (rtol * np.abs(b) + atol_rel * max(scale, 1e-300) + 1e-300)))
+
+
+def dump_outputs(dump_dir, workload, read):
+    """--dump-outputs: read(p) is output p of the last timed step; written as DIR/<workload>_<p>.npy (float64).  An output
+    longer than DUMP_MAX_ENTRIES is sampled at seeded positions that depend only on its length, so two builds of the same
+    workload keep the same entries."""
+    os.makedirs(dump_dir, exist_ok=True)
+    for p in PROGS:
+        a = np.asarray(read(p), dtype=np.float64).ravel()
+        if a.size > DUMP_MAX_ENTRIES:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ENTRIES, replace=False))]
+        np.save(os.path.join(dump_dir, "%s_%s.npy" % (workload, p)), a)
 
 
 def load_traffic(workload, kname):
@@ -452,6 +470,8 @@ def bench_single(name, args, grp, hbm_peak, peak_src):
     solo = Group(0, 1, grp.local_rank)
     ms, E, clocks = timed_device(lambda n: o.run_device(PROGS, n), solo, args.steps, args.warmup, grp.local_rank)
     launches = o.kernel_launches() - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, name, o.read_output)
     per_eval_ms = ms / (args.steps * E)
     sys.stderr.write("[bench] %s device: %.4f ms/eval (%d evals per step)\n" % (name, per_eval_ms, E))
     sb = survey_bytes(name, sizes)
@@ -573,7 +593,7 @@ def bench_c3_sharded(args, grp, hbm_peak, peak_src):
             t0 = time.perf_counter()
             five(2), five(3)
             probe = (time.perf_counter() - t0) / 2.0
-            E2 = max(1, int(math.ceil(TARGET_E2E_S / (args.steps * max(probe, 1e-6)))))
+            E2 = max(1, int(math.ceil(TARGET_E2E_STEP_S / max(probe, 1e-6))))
             t0 = time.perf_counter()
             for i in range(args.steps * E2):
                 five(i)
@@ -664,18 +684,19 @@ def bench_multistart(args, grp, hbm_peak, peak_src):
     l0 = o.kernel_launches()
     ms, E, clocks = timed_device(lambda m_: o.run_device(PROGS, m_), grp, args.steps, args.warmup, grp.local_rank)
     launches = o.kernel_launches() - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "c4", o.read_output)
     e2e = None
     if not args.device_only:
         o.eval(X[b0:b1], LAM, SIG)
         grp.barrier()
-        e_steps = max(1, min(args.steps, 3))
         t0 = time.perf_counter()
-        for _ in range(e_steps):
+        for _ in range(args.steps):
             o.eval(X[b0:b1], LAM, SIG)
         dt = float(grp.max([time.perf_counter() - t0])[0])
-        e2e = {"value": Btot * e_steps / dt, "unit": "evals/s", "api": "BatchedOracles.eval (host arrays in/out)",
+        e2e = {"value": Btot * args.steps / dt, "unit": "evals/s", "api": "BatchedOracles.eval (host arrays in/out)",
                "h2d_bytes_per_step": int(8 * Btot * (n + k + 1)),
-               "d2h_bytes_per_step": int(8 * Btot * (1 + n + k + o.nnz_jac + o.nnz_hess)), "steps": e_steps}
+               "d2h_bytes_per_step": int(8 * Btot * (1 + n + k + o.nnz_jac + o.nnz_hess)), "steps": args.steps}
     res = None
     if rank == 0:
         per = o.profile_instrs("all", iters=2)
@@ -759,11 +780,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--device-only", action="store_true",
                     help="profiling aid: only the device-resident step loop and the per-instruction timing")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed device step as DIR/<workload>_<output>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs --impl ours in one process (WORLD_SIZE=1)")
     headline = "c3" if args.workload == "all" else args.workload
     subs = [w for w in os.environ.get("DNLP_BENCH_SUBS", "c4,c2,c5").split(",") if w] if args.workload == "all" else []
 

@@ -54,7 +54,7 @@ EXPORTS = [
     "dnlp_host_alloc", "dnlp_host_free", "dnlp_upload_point", "dnlp_run_device", "dnlp_profile_instrs",
     "dnlp_read_output", "dnlp_kernel_launches", "dnlp_set_cache", "dnlp_set_graphs", "dnlp_set_parallel", "dnlp_set_windows", "dnlp_set_dynamic", "dnlp_eval_dyn", "dnlp_bind_outputs", "dnlp_set_params", "dnlp_instr_kernel", "dnlp_run", "dnlp_output_ptr",
     "dnlp_batch_create", "dnlp_batch_destroy", "dnlp_batch_last_error", "dnlp_batch_eval", "dnlp_batch_upload",
-    "dnlp_batch_run_device", "dnlp_batch_profile_instrs", "dnlp_batch_kernel_launches", "dnlp_batch_profile_groups",
+    "dnlp_batch_run_device", "dnlp_batch_read_output", "dnlp_batch_profile_instrs", "dnlp_batch_kernel_launches", "dnlp_batch_profile_groups",
     "dnlp_comm_unique_id", "dnlp_comm_create", "dnlp_comm_destroy", "dnlp_comm_last_error", "dnlp_comm_has_nccl",
     "dnlp_comm_ipc_handle", "dnlp_comm_open_peers", "dnlp_comm_allreduce_host",
     "dnlp_shard_create", "dnlp_shard_destroy", "dnlp_shard_last_error", "dnlp_shard_set_output",
@@ -126,6 +126,7 @@ def lib():
     L.dnlp_batch_eval.argtypes = [vp] + [c_f64p] * 8
     L.dnlp_batch_upload.argtypes = [vp, c_f64p, c_f64p, c_f64p]
     L.dnlp_batch_run_device.argtypes = [vp, C.c_int32, C.c_int32, c_f32p]
+    L.dnlp_batch_read_output.argtypes = [vp, C.c_int32, c_f64p]
     L.dnlp_batch_profile_instrs.argtypes = [vp, C.c_int32, C.c_int32, c_f32p]
     L.dnlp_batch_profile_groups.argtypes = [vp, C.c_int32, c_f32p, c_f64p, C.c_int32]
     L.dnlp_batch_kernel_launches.argtypes = [vp]

@@ -498,6 +498,16 @@ int dnlp_batch_run_device(dnlp_batch *o, int32_t prog_mask, int32_t iters, float
   return 0;
 }
 
+int dnlp_batch_read_output(dnlp_batch *o, int32_t space, double *out) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  CKB(cudaSetDevice(o->device));
+  if (space < 1 || space > 5) { err = "bad output id"; return 1; }
+  if (o->get(space, out)) return 1;
+  CKB(cudaStreamSynchronize(o->stream));
+  return 0;
+}
+
 int dnlp_batch_profile_instrs(dnlp_batch *o, int32_t p, int32_t iters, float *ms_per_instr) {
   if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
   std::string &err = o->err;

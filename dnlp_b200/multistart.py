@@ -76,6 +76,13 @@ class BatchedOracles:
         self.dev.check(self.dev._L.dnlp_batch_run_device(self.dev.h, mask, int(iters), C.byref(ms)))
         return float(ms.value)
 
+    def read_output(self, name):
+        """The device output ``name`` as a (B, len) array, as the last ``run_device`` step left it."""
+        out = np.empty((self.batch, self._len[name]))
+        space = {"f": 1, "grad": 2, "g": 3, "jac": 4, "hess": 5}[name]
+        self.dev.check(self.dev._L.dnlp_batch_read_output(self.dev.h, space, _ptr(out)))
+        return out
+
     def profile_instrs(self, program="all", iters=3):
         out = np.zeros(max(len(self.tape.instrs), 1), dtype=np.float32)
         self.dev.check(self.dev._L.dnlp_batch_profile_instrs(self.dev.h, _cabi.PROG_IDS[program], int(iters),

@@ -193,6 +193,7 @@ int dnlp_batch_eval(dnlp_batch *b, const double *X, const double *LAM, const dou
                     double *F, double *GRAD, double *G, double *JAC, double *HESS);
 int dnlp_batch_upload(dnlp_batch *b, const double *X, const double *LAM, const double *SIGMA);
 int dnlp_batch_run_device(dnlp_batch *b, int32_t prog_mask, int32_t iters, float *elapsed_ms);
+int dnlp_batch_read_output(dnlp_batch *b, int32_t dst_space, double *out);   /* D2H of one output, start-major */
 int dnlp_batch_profile_instrs(dnlp_batch *b, int32_t prog, int32_t iters, float *ms_per_instr);
 int dnlp_batch_profile_groups(dnlp_batch *b, int32_t iters, float *ms_per_group, double *flops_per_group,
                               int32_t max_groups);   /* grouped DMMA GEMM launches, timed with CUDA events */

@@ -86,6 +86,7 @@ class _InterpLib:
 
     # ---- measurement hooks of bench.py: no device, so no timings - fixed figures that keep the control flow going ----
     def dnlp_upload_point(self, h, x, lam, sigma):
+        self.x = np.array(_arr(x, self.n), copy=True)
         self.lam = np.zeros(self.m) if not lam else np.array(_arr(lam, self.m), copy=True)
         self.sigma, self.launches = float(sigma), getattr(self, "launches", 0)
         return 0
@@ -107,7 +108,9 @@ class _InterpLib:
         return b"tape_interpreter"
 
     def dnlp_read_output(self, h, space, out):
-        return 1
+        # what dnlp_run_device left on the device: the outputs at the uploaded point
+        _arr(out, self.len[int(space)])[:] = self._eval(int(space), self.x)
+        return 0
 
     def dnlp_set_graphs(self, h, on):
         return 0
@@ -148,11 +151,15 @@ class _InterpBatchLib:
     def _mat(self, ptr, cols):
         return None if not ptr else np.ctypeslib.as_array(ptr, shape=(self.B * max(int(cols), 1),))[:self.B * int(cols)].reshape(self.B, int(cols))
 
+    def _inputs(self, X, LAM, SIGMA):
+        return (self._mat(X, self.n), self._mat(LAM, self.m) if self.m else None,
+                None if not SIGMA else np.ctypeslib.as_array(SIGMA, shape=(self.B,)))
+
     def dnlp_batch_eval(self, h, X, LAM, SIGMA, f, grad, g, jac, hess):
-        X = self._mat(X, self.n)
-        LAM = self._mat(LAM, self.m) if self.m else None
-        SIG = None if not SIGMA else np.ctypeslib.as_array(SIGMA, shape=(self.B,))
         outs = {k: self._mat(p, self.len[k]) for k, p in (("f", f), ("grad", grad), ("g", g), ("jac", jac), ("hess", hess))}
+        return self._fill(*self._inputs(X, LAM, SIGMA), outs)
+
+    def _fill(self, X, LAM, SIG, outs):
         with np.errstate(all="ignore"):
             for b in range(self.B):
                 for k, out in outs.items():
@@ -166,7 +173,13 @@ class _InterpBatchLib:
         return 0
 
     def dnlp_batch_upload(self, h, X, LAM, SIGMA):
+        self.uploaded = [None if a is None else np.array(a, copy=True) for a in self._inputs(X, LAM, SIGMA)]
         return 0
+
+    def dnlp_batch_read_output(self, h, space, out):
+        # what dnlp_batch_run_device left on the device: the outputs at the uploaded points
+        name = _NAME[int(space)]
+        return self._fill(*self.uploaded, {name: self._mat(out, self.len[name])})
 
     def dnlp_batch_run_device(self, h, mask, iters, ms_out):
         self.launches += int(iters) * len(self.tape.programs["all"])

@@ -21,9 +21,9 @@ def test_single_gpu_bench_line(workload, scale, monkeypatch):
     from dnlp_b200 import _cabi
     host_logic_device.install(monkeypatch)
     monkeypatch.setattr(_cabi, "device_synchronize", lambda *a: None)
-    monkeypatch.setattr(bench, "TARGET_E2E_S", 0.05)
+    monkeypatch.setattr(bench, "TARGET_E2E_STEP_S", 0.05 / 3)
     args = argparse.Namespace(gpus=1, steps=3, warmup=3, workload=workload, scale=scale, impl="ours", no_cpu_baseline=True,
-                              device_only=False)
+                              device_only=False, dump_outputs=None)
     grp = bench.Group(0, 1, 0)
     res = bench.bench_single(workload, args, grp, 6545.0, "test")
     for key in ("value", "unit", "ms_per_step", "evals_per_step", "ms_per_eval", "config", "clocks", "gpu_launches", "e2e",
@@ -55,10 +55,10 @@ def test_multistart_bench_line_and_batched_oracles(monkeypatch):
     from oracle.dnlp_oracle import RefOracles
     host_logic_device.install(monkeypatch)
     monkeypatch.setattr(_cabi, "device_synchronize", lambda *a: None)
-    monkeypatch.setattr(bench, "TARGET_E2E_S", 0.05)
+    monkeypatch.setattr(bench, "TARGET_E2E_STEP_S", 0.05 / 3)
     monkeypatch.setenv("DNLP_C4_BATCH", "6")
     args = argparse.Namespace(gpus=1, steps=3, warmup=3, workload="c4", scale=0.05, impl="ours", no_cpu_baseline=True,
-                              device_only=False)
+                              device_only=False, dump_outputs=None)
     res = bench.bench_multistart(args, bench.Group(0, 1, 0), 6545.0, "test")
     for key in ("value", "unit", "ms_per_step", "config", "gpu_launches", "e2e", "roofline"):
         assert key in res, key
@@ -86,3 +86,48 @@ def test_multistart_bench_line_and_batched_oracles(monkeypatch):
     with pytest.raises(ValueError):
         bo.eval(X, want=("hess",))
     bo.close()
+
+
+def _device_args(workload, scale, steps, dump=None):
+    return argparse.Namespace(gpus=1, steps=steps, warmup=3, workload=workload, scale=scale, impl="ours", no_cpu_baseline=True,
+                              device_only=True, dump_outputs=dump)
+
+
+def test_steps_sets_the_number_of_timed_steps(monkeypatch):
+    """--steps K times K steps of one size (the stand-in reports 0.05 ms per evaluation): twice the steps, the same
+    step, twice the evaluations in the timed window.  The batched e2e leg runs K steps as well."""
+    import bench
+    from dnlp_b200 import _cabi
+    host_logic_device.install(monkeypatch)
+    monkeypatch.setattr(_cabi, "device_synchronize", lambda *a: None)
+    res = {k: bench.bench_single("c1", _device_args("c1", 1.0, k), bench.Group(0, 1, 0), 6545.0, "test") for k in (3, 6)}
+    assert res[3]["evals_per_step"] == res[6]["evals_per_step"] == round(bench.TARGET_STEP_S * 1e3 / 0.05)
+    for k, r in res.items():
+        assert r["ms_per_step"] == pytest.approx(0.05 * r["evals_per_step"])
+        assert r["value"] == pytest.approx(k * r["evals_per_step"] / (k * r["ms_per_step"] * 1e-3))
+    monkeypatch.setenv("DNLP_C4_BATCH", "3")
+    args = argparse.Namespace(gpus=1, steps=4, warmup=3, workload="c4", scale=0.05, impl="ours", no_cpu_baseline=True,
+                              device_only=False, dump_outputs=None)
+    assert bench.bench_multistart(args, bench.Group(0, 1, 0), 6545.0, "test")["e2e"]["steps"] == 4
+
+
+@pytest.mark.parametrize("workload,scale", [("c3", 0.002), ("c4", 0.05)])
+def test_dump_outputs_are_the_last_timed_step(workload, scale, tmp_path, monkeypatch):
+    """--dump-outputs writes the five outputs of the device-resident path at the bench's own seeded inputs, float64;
+    an output longer than DUMP_MAX_ENTRIES is sampled at seeded positions that depend only on its length."""
+    import bench
+    from dnlp_b200 import _cabi
+    from golden_util import assert_close
+    from workload_cases import bench_dump_expected
+    host_logic_device.install(monkeypatch)
+    monkeypatch.setattr(_cabi, "device_synchronize", lambda *a: None)
+    monkeypatch.setattr(bench, "DUMP_MAX_ENTRIES", 64)
+    monkeypatch.setenv("DNLP_C4_BATCH", "3")
+    run = bench.bench_multistart if workload == "c4" else (lambda a, *r: bench.bench_single(workload, a, *r))
+    run(_device_args(workload, scale, 2, dump=str(tmp_path)), bench.Group(0, 1, 0), 6545.0, "test")
+    want = bench_dump_expected(workload, scale, 64)
+    assert sorted(os.listdir(tmp_path)) == sorted("%s_%s.npy" % (workload, p) for p in bench.PROGS)
+    for p in bench.PROGS:
+        got = np.load(tmp_path / ("%s_%s.npy" % (workload, p)))
+        assert got.dtype == np.float64 and got.size <= 64
+        assert_close(got, want[p], p, atol=1e-9 if p == "g" else 1e-12)

@@ -1,19 +1,14 @@
 """Batched best_of (SURVEY 8f item 1; reference loop: cvxpy/problems/problem.py:1249-1275, objective set:
 ipopt_nlpif.py:87-89).  All starts advance in lock step over one compiled tape; the per-start results must be
 the serial loop's, start by start."""
-import os
-import sys
-import types
-
 import numpy as np
 import pytest
 
 import kkt_newton
 from dnlp_b200 import workloads as W
 from dnlp_b200.best_of import best_of_lockstep, lockstep_newton_kkt
+from oracle import ref_driver as R
 from oracle.dnlp_oracle import RefOracles
-
-REF = "/root/reference"
 
 
 class CpuBatch:
@@ -61,18 +56,12 @@ def test_lockstep_equals_serial_newton_start_by_start():
     assert out["best"] == int(np.argmin(out["all_objs"]))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "cvxpy")), reason="reference not present")
+@pytest.mark.skipif(not R.available(), reason="reference not present (oracle/_ref)")
 def test_solve_best_of_reproduces_the_reference_loop():
     """The reference's loop, emulated with the stand-in solver (IPOPT is not installed): same sampler stream,
     chain re-applied per start, one solve per start.  solve_best_of must return the same objective set, the
     same best value, and leave them where the reference leaves them (extra_stats)."""
-    v = types.ModuleType("cvxpy.version")
-    v.short_version = v.version = "1.8.0"
-    v.full_version, v.git_revision, v.commit_count, v.release = "1.8.0.dev0", "Unknown", "0", False
-    sys.modules.setdefault("cvxpy.version", v)
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import cvxpy as cp
+    cp = R.load_reference()
     from cvxpy.reductions.cvx_attr2constr import CvxAttr2Constr
     from cvxpy.reductions.dnlp2smooth.dnlp2smooth import Dnlp2Smooth
     from cvxpy.reductions.flip_objective import FlipObjective

@@ -717,3 +717,26 @@ def test_gpu_parameter_sweep_without_recompiling(eager, gpu_mod):
             o.set_parameters(np.zeros(3))
     finally:
         o.close()
+
+
+@pytest.mark.parametrize("workload,scale", [("c3", 0.002), ("c4", 0.05)])
+def test_gpu_bench_dump_outputs_are_the_last_device_step(workload, scale, tmp_path, monkeypatch):
+    """bench.py --dump-outputs on the device: what the timed device steps left in HBM, read back after the timed
+    window, equals the CPU oracle at the bench's seeded inputs (single oracle and batched multi-start path)."""
+    import argparse
+    import os
+
+    import bench
+    from workload_cases import bench_dump_expected
+    monkeypatch.setattr(bench, "DUMP_MAX_ENTRIES", 4096)
+    monkeypatch.setenv("DNLP_C4_BATCH", "5")
+    args = argparse.Namespace(gpus=1, steps=2, warmup=3, workload=workload, scale=scale, impl="ours", no_cpu_baseline=True,
+                              device_only=True, dump_outputs=str(tmp_path))
+    run = bench.bench_multistart if workload == "c4" else (lambda a, *r: bench.bench_single(workload, a, *r))
+    run(args, bench.Group(0, 1, 0), 6545.0, "test")
+    want = bench_dump_expected(workload, scale, 4096)
+    assert sorted(os.listdir(tmp_path)) == sorted("%s_%s.npy" % (workload, p) for p in bench.PROGS)
+    for p in bench.PROGS:
+        got = np.load(tmp_path / ("%s_%s.npy" % (workload, p)))
+        assert got.dtype == np.float64
+        assert_close(got, want[p], p, atol=1e-9 if p == "g" else 1e-12)

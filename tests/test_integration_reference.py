@@ -1,31 +1,22 @@
-"""Drop-in boundary against the LIVE reference (runs only where /root/reference exists).
+"""Drop-in boundary against the LIVE reference (runs only where oracle/make_ref.sh has installed it as oracle/_ref).
 
 `install()` rebinds the one name the reference's solver interface instantiates; the reduction
 chain then yields a GpuOracles object whose structures equal the reference Oracles' bit for bit.
 The device upload is stubbed here (no GPU in the build container); the CUDA path itself is
 covered by tests/test_gpu_parity.py."""
-import os
-import sys
 import types
 
 import numpy as np
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "cvxpy")), reason="reference not present")
+from oracle import ref_driver as R
+
+pytestmark = pytest.mark.skipif(not R.available(), reason="reference not present (oracle/_ref)")
 
 
 @pytest.fixture(scope="module")
 def cp():
-    v = types.ModuleType("cvxpy.version")
-    v.short_version = v.version = "1.8.0"
-    v.full_version, v.git_revision, v.commit_count, v.release = "1.8.0.dev0", "Unknown", "0", False
-    sys.modules["cvxpy.version"] = v
-    sys.path.insert(0, REF)
-    sys.dont_write_bytecode = True
-    import cvxpy
-    yield cvxpy
-    sys.path.remove(REF)
+    return R.load_reference()
 
 
 def _chain(cp, prob):

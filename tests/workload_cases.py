@@ -53,3 +53,36 @@ class MediumGolden:
         assert (len(jr), len(hr)) == (self.nnz_jac, self.nnz_hess)
         for name, arr in (("jac_rows", jr), ("jac_cols", jc), ("hess_rows", hr), ("hess_cols", hc)):
             assert digest(arr) == str(self.z[name + "_sha256"]), "%s differs from the reference's" % name
+
+
+def bench_dump_expected(workload, scale, max_entries):
+    """What ``bench.py --dump-outputs`` must write for ``workload`` at ``scale`` (c4: DNLP_C4_BATCH starts): the CPU
+    oracle port at the bench's seeded inputs, sampled as the bench samples an output longer than ``max_entries``."""
+    import bench
+    from oracle.dnlp_oracle import RefOracles
+    if workload == "c4":
+        s = bench.sizes_of("c4", scale)
+        P, q, rng = W.qcqp_data(s["n"], s["k"])
+        prob = W.qcqp(P, q)
+        B = int(os.environ["DNLP_C4_BATCH"])
+        X = rng.uniform(-1, 1, (B, s["n"]))
+        LAM = np.random.default_rng(17).standard_normal((B, s["k"]))
+        points = [(X[b], LAM[b], 1.0) for b in range(B)]
+    else:
+        prob = bench.build_workload(workload, scale)
+        points = [bench.eval_point(prob, 0)]
+    ref = RefOracles(prob)
+    ref.jacobianstructure(), ref.hessianstructure()
+    vals = {p: [] for p in bench.PROGS}
+    with np.errstate(all="ignore"):
+        for x, lam, sigma in points:
+            for p, v in zip(bench.PROGS, (ref.objective(x), ref.gradient(x), ref.constraints(x), ref.jacobian(x),
+                                          ref.hessian(x, lam, sigma))):
+                vals[p].append(np.array(v, dtype=np.float64).ravel())
+    out = {}
+    for p, v in vals.items():
+        a = np.concatenate(v)
+        if a.size > max_entries:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, max_entries, replace=False))]
+        out[p] = a
+    return out
