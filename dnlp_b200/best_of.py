@@ -11,8 +11,8 @@ compile once (dnlp_b200/compile_cache.py); here the N solves themselves are batc
     Hess L of every start (csrc/dnlp_batch.cu); the B dense KKT systems are solved as one batched LAPACK
     call on the host.  It touches the oracle only through the callback outputs and structures, like the
     test-suite's serial stand-in for IPOPT (tests/kkt_newton.py), and takes exactly its iterates.
-    It is NOT an interior-point method: inequality constraints and active bounds are outside its scope
-    (use ``solve_best_of(..., solver="ipopt")`` for those: per-start IPOPT instances, still one tape).
+    It is NOT an interior-point method: problems with a finite variable bound or an inequality row go to
+    ``lockstep_ipm`` (dnlp_b200/lockstep_ipm.py) instead, whose B KKT systems are factored on the GPU.
 
 ``solve_best_of``  the reference's loop with the solves batched: N initial points from the reference's own
     sampler, one compile, one lock-step solve, ``all_objs_from_best_of`` and the best start unpacked through
@@ -75,16 +75,34 @@ def lockstep_newton_kkt(ev, X0, tol=1e-12, max_iter=60):
             "converged": done}
 
 
-def best_of_lockstep(problem_ir, X0, device=0, evaluator=None, tol=1e-12, max_iter=60):
+def _equality_only(problem_ir):
+    """No finite variable bound and no inequality row: the problem the Newton-KKT iteration handles."""
+    finite = [v is not None and np.any(np.isfinite(v)) for v in (problem_ir.lb, problem_ir.ub)]
+    cl, cu = problem_ir.cl, problem_ir.cu
+    two_sided = problem_ir.m > 0 and (cl is None or cu is None or np.any(np.asarray(cl) != np.asarray(cu)))
+    return not any(finite) and not two_sided
+
+
+def best_of_lockstep(problem_ir, X0, device=0, evaluator=None, kkt=None, tol=None, max_iter=None):
     """All starts ``X0`` (B, n) of one smooth problem in lock step on the GPU; ``evaluator`` replaces
-    ``BatchedOracles`` (CPU tests).  Adds ``all_objs`` and ``best`` (index of the smallest objective among
-    the converged starts) to the solver's result."""
+    ``BatchedOracles`` (CPU tests).  Equality-constrained problems without bounds take ``lockstep_newton_kkt``
+    (defaults tol 1e-12, 60 iterations), every other problem ``lockstep_ipm`` (tol 1e-8, 500 iterations) with the KKT
+    backend ``kkt`` (default: ``DeviceKKT`` on the evaluator).  Adds ``all_objs`` and ``best`` (index of the smallest
+    objective among the converged starts) to the solver's result."""
     own = evaluator is None
     if own:
         from .multistart import BatchedOracles
         evaluator = BatchedOracles(problem_ir, len(X0), device=device)
     try:
-        out = lockstep_newton_kkt(evaluator, X0, tol=tol, max_iter=max_iter)
+        if _equality_only(problem_ir):
+            out = lockstep_newton_kkt(evaluator, X0, tol=1e-12 if tol is None else tol,
+                                      max_iter=60 if max_iter is None else max_iter)
+        else:
+            from .lockstep_ipm import DeviceKKT, lockstep_ipm
+            out = lockstep_ipm(evaluator, DeviceKKT(evaluator) if kkt is None else kkt, X0, lb=problem_ir.lb,
+                               ub=problem_ir.ub, cl=problem_ir.cl, cu=problem_ir.cu, tol=1e-8 if tol is None else tol,
+                               max_iter=500 if max_iter is None else max_iter)
+            out["converged"] = out["status"] == 0
     finally:
         if own:
             evaluator.close()
@@ -101,12 +119,15 @@ def _pick(smooth_objs, maximize, faithful):
     return int(np.argmin(smooth_objs))
 
 
-def solve_best_of(prob, best_of, solver="lockstep", device=0, evaluator_factory=None, faithful=True, **solver_opts):
+def solve_best_of(prob, best_of, solver="lockstep", device=0, evaluator_factory=None, faithful=True, kkt_factory=None,
+                  **solver_opts):
     """The reference's ``best_of`` loop (problem.py:1249-1275) with one compile and batched solves.
     ``prob`` is a cvxpy Problem of the installed reference; returns ``prob.value`` and leaves variable values,
     ``prob.solver_stats.extra_stats['all_objs_from_best_of']`` exactly where the reference's loop leaves them.
-    ``solver``: "lockstep" (equality-constrained problems, all starts at once on the GPU) or "ipopt"
-    (per-start ``solve_via_data`` on the shared resident oracle; needs cyipopt).
+    ``solver``: "lockstep" (all starts at once on the GPU: the Newton-KKT iteration for equality-constrained problems
+    without bounds, the lock-step interior-point method for every other problem) or "ipopt" (per-start
+    ``solve_via_data`` on the shared resident oracle; needs cyipopt).  ``evaluator_factory(problem_ir, B)`` and
+    ``kkt_factory(evaluator)`` replace ``BatchedOracles`` and the device KKT backend (CPU tests).
 
     ``faithful`` (default): the reference's loop ranks the starts by ``self.objective.value`` with ``<`` whatever the
     sense (problem.py:1262-1268), so for a Maximize problem it keeps the start with the SMALLEST objective, and it
@@ -142,17 +163,20 @@ def solve_best_of(prob, best_of, solver="lockstep", device=0, evaluator_factory=
         best = _pick(objs, maximize, faithful)
         best_solution = sols[best]
     else:
-        if np.any(np.asarray(data["cu"]) != np.asarray(data["cl"])) or np.any(np.isfinite(data["lb"])) \
-                or np.any(np.isfinite(data["ub"])):
-            raise NotImplementedError("the lock-step Newton-KKT driver handles equality constraints without variable "
-                                      "bounds; use solver='ipopt' for this problem")
         pir = data_to_ir(data)
         ev = evaluator_factory(pir, best_of) if evaluator_factory is not None else None
-        out = best_of_lockstep(pir, np.stack(starts), device=device, evaluator=ev, **solver_opts)
+        kkt = kkt_factory(ev) if (kkt_factory is not None and ev is not None) else None
+        out = best_of_lockstep(pir, np.stack(starts), device=device, evaluator=ev, kkt=kkt, **solver_opts)
         objs = out["all_objs"]
         best = _pick(np.asarray(objs), maximize, faithful)
-        best_solution = {"status": 0 if out["converged"][best] else -1, "x": out["x"][best], "obj_val": float(objs[best]),
-                         "mult_g": out["lam"][best], "iterations": int(out["iterations"][best])}
+        if "status" in out:            # the interior-point driver: IPOPT's status codes and bound multipliers
+            best_solution = {"status": int(out["status"][best]), "x": out["x"][best], "obj_val": float(objs[best]),
+                             "mult_g": out["lam"][best], "mult_x_L": out["zL"][best], "mult_x_U": out["zU"][best],
+                             "iterations": int(out["iterations"][best])}
+        else:
+            best_solution = {"status": 0 if out["converged"][best] else -1, "x": out["x"][best],
+                             "obj_val": float(objs[best]), "mult_g": out["lam"][best],
+                             "iterations": int(out["iterations"][best])}
     true_objs = -np.asarray(objs) if maximize else np.asarray(objs)      # self.objective.value at every start's solution
     all_objs = -true_objs if (maximize and faithful) else true_objs
     best_solution["all_objs_from_best_of"] = all_objs

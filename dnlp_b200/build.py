@@ -9,7 +9,7 @@ LIB = os.path.join(PKG, "libdnlp_b200.so")
 SOURCES = [os.path.join(PKG, "csrc", "dnlp_cabi.cu"), os.path.join(PKG, "csrc", "dnlp_batch.cu"),
            os.path.join(PKG, "csrc", "dnlp_shard.cu")]
 HEADERS = [os.path.join(PKG, "csrc", "dnlp_kernels.cuh"), os.path.join(PKG, "csrc", "dnlp_engine.h"), os.path.join(PKG, "csrc", "dnlp_batch_kernels.cuh"),
-           os.path.join(ROOT, "include", "dnlp_b200.h")]
+           os.path.join(PKG, "csrc", "dnlp_batch_kkt.cuh"), os.path.join(ROOT, "include", "dnlp_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC,-fopenmp", "-Xptxas", "-v", "-lgomp", "-ldl"]
 

@@ -2,9 +2,12 @@
 // See include/dnlp_b200.h (dnlp_batch_*) and dnlp_batch_kernels.cuh.
 #include "../../include/dnlp_b200.h"
 #include "dnlp_batch_kernels.cuh"
+#include "dnlp_batch_kkt.cuh"
 
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <map>
 #include <string>
 #include <vector>
 
@@ -51,6 +54,19 @@ struct dnlp_batch {
   std::vector<void *> owned;
   int64_t launches = 0;
   std::string err;
+  // dense KKT systems of the lock-step interior-point driver (dnlp_batch_kkt_*); slot b of every array is start b
+  struct Kkt {
+    int64_t N = 0, M = 0, ntgt = 0, nnzH = 0;
+    int32_t *ti = nullptr, *tj = nullptr, *sp = nullptr, *src = nullptr;   // targets and their sources, pattern order
+    double *K = nullptr, *Dg = nullptr, *Wd = nullptr, *work = nullptr;
+    double *sigma = nullptr, *dw = nullptr, *dc = nullptr, *rhs = nullptr, *sol = nullptr, *wq = nullptr;
+    int32_t *starts = nullptr, *inertia = nullptr;
+    std::vector<void *> owned;
+  } kkt;
+  void kkt_free() {
+    for (void *p : kkt.owned) cudaFree(p);
+    kkt = Kkt();
+  }
 
   template <typename T>
   int upload(const T *host, int64_t count, T **dev) {
@@ -291,6 +307,7 @@ void dnlp_batch_destroy(dnlp_batch *o) {
   cudaSetDevice(o->device);
   if (o->stream) cudaStreamSynchronize(o->stream);
   for (auto &g : o->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
+  o->kkt_free();
   for (void *p : o->owned) cudaFree(p);
   if (o->ev0) cudaEventDestroy(o->ev0);
   if (o->ev1) cudaEventDestroy(o->ev1);
@@ -559,5 +576,146 @@ int dnlp_batch_profile_groups(dnlp_batch *o, int32_t iters, float *ms_per_group,
 }
 
 int64_t dnlp_batch_kernel_launches(dnlp_batch *o) { return o ? o->launches : -1; }
+
+int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                         const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  CKB(cudaSetDevice(o->device));
+  CKB(cudaStreamSynchronize(o->stream));
+  o->kkt_free();
+  const int64_t n = o->n, m = o->m, nnzJ = o->out_len[4], nnzH = o->out_len[5];
+  if (ns < 0 || ns > m) { err = "kkt_setup: the number of slack rows must lie in [0, m]"; return 1; }
+  const int64_t N = n + ns, M = N + m, B = o->B;
+  // the scatter map: every lower-triangle target (i, j) of K with its sources in pattern order
+  std::map<int64_t, std::vector<int32_t>> tgt;
+  for (int64_t i = 0; i < M; ++i) tgt[i * M + i];
+  std::vector<char> seen(m > 0 ? m : 1, 0);
+  for (int64_t s = 0; s < ns; ++s) {
+    const int32_t r = slack_rows[s];
+    if (r < 0 || r >= m || seen[r]) { err = "kkt_setup: slack rows must be distinct constraint rows"; return 1; }
+    seen[r] = 1;
+  }
+  for (int64_t k = 0; k < nnzH; ++k) {
+    const int64_t r = hess_rows[k], c = hess_cols[k];
+    if (r < 0 || r >= n || c < 0 || c >= n) { err = "kkt_setup: Hessian pattern entry out of range"; return 1; }
+    tgt[std::max(r, c) * M + std::min(r, c)].push_back((int32_t)k);
+  }
+  for (int64_t k = 0; k < nnzJ; ++k) {
+    const int64_t r = jac_rows[k], c = jac_cols[k];
+    if (r < 0 || r >= m || c < 0 || c >= n) { err = "kkt_setup: Jacobian pattern entry out of range"; return 1; }
+    tgt[(N + r) * M + c].push_back((int32_t)(nnzH + k));
+  }
+  for (int64_t s = 0; s < ns; ++s) tgt[(N + slack_rows[s]) * M + n + s].push_back(-1);
+  std::vector<int32_t> ti, tj, sp(1, 0), src;
+  for (auto &kv : tgt) {
+    ti.push_back((int32_t)(kv.first / M));
+    tj.push_back((int32_t)(kv.first % M));
+    src.insert(src.end(), kv.second.begin(), kv.second.end());
+    sp.push_back((int32_t)src.size());
+  }
+  // refuse what does not fit: the B dense systems dominate
+  const double kbytes = (double)B * (double)M * (double)M * 8.0;
+  const double vbytes = (double)B * (double)(9 * M + 2 * N + 4) * 8.0 + (double)(3 * ti.size() + src.size() + 1) * 4.0;
+  size_t free_b = 0, total_b = 0;
+  CKB(cudaMemGetInfo(&free_b, &total_b));
+  if (kbytes + vbytes > 0.95 * (double)free_b) {
+    char buf[320];
+    snprintf(buf, sizeof buf, "kkt_setup: the dense KKT systems need B*(N+m)^2*8 = %lld*%lld^2*8 = %.3e bytes "
+             "(+%.3e for vectors) but the device has %.3e bytes free; use fewer starts per batch",
+             (long long)B, (long long)M, kbytes, vbytes, (double)free_b);
+    err = buf;
+    return 1;
+  }
+  auto &Q = o->kkt;
+  Q.N = N; Q.M = M; Q.ntgt = (int64_t)ti.size(); Q.nnzH = nnzH;
+  auto alloc = [&](size_t bytes, void **p) -> int {
+    CKB(cudaMalloc(p, bytes < 8 ? 8 : bytes));
+    Q.owned.push_back(*p);
+    return 0;
+  };
+  auto up = [&](const std::vector<int32_t> &h, int32_t **d) -> int {
+    if (alloc(h.size() * sizeof(int32_t), (void **)d)) return 1;
+    CKB(cudaMemcpyAsync(*d, h.data(), h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, o->stream));
+    return 0;
+  };
+  if (up(ti, &Q.ti) || up(tj, &Q.tj) || up(sp, &Q.sp) || up(src, &Q.src)) { o->kkt_free(); return 1; }
+  if (alloc((size_t)B * M * M * 8, (void **)&Q.K) || alloc((size_t)B * M * 8, (void **)&Q.Dg) ||
+      alloc((size_t)B * N * 8, (void **)&Q.Wd) || alloc((size_t)B * 3 * M * 8, (void **)&Q.work) ||
+      alloc((size_t)B * N * 8, (void **)&Q.sigma) || alloc((size_t)B * 8, (void **)&Q.dw) ||
+      alloc((size_t)B * 8, (void **)&Q.dc) || alloc((size_t)B * M * 8, (void **)&Q.rhs) ||
+      alloc((size_t)B * M * 8, (void **)&Q.sol) || alloc((size_t)B * 8, (void **)&Q.wq) ||
+      alloc((size_t)B * 4, (void **)&Q.starts) || alloc((size_t)B * 3 * 4, (void **)&Q.inertia)) {
+    o->kkt_free();
+    return 1;
+  }
+  CKB(cudaStreamSynchronize(o->stream));
+  return 0;
+}
+
+int dnlp_batch_kkt_solve(dnlp_batch *o, int32_t count, const int32_t *starts, const double *sigma, const double *dw,
+                         const double *dc, const double *rhs, double *sol, int32_t *inertia, double *wquad,
+                         float *elapsed_ms) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  auto &Q = o->kkt;
+  if (Q.M == 0) { err = "kkt_solve: call dnlp_batch_kkt_setup first"; return 1; }
+  if (count < 0 || count > o->B) { err = "kkt_solve: count must lie in [0, batch]"; return 1; }
+  if (count == 0) { if (elapsed_ms) *elapsed_ms = 0.f; return 0; }
+  std::vector<char> seen(o->B, 0);
+  for (int c = 0; c < count; ++c) {
+    if (starts[c] < 0 || starts[c] >= o->B || seen[starts[c]]) { err = "kkt_solve: start ids must be distinct and in [0, batch)"; return 1; }
+    seen[starts[c]] = 1;
+  }
+  CKB(cudaSetDevice(o->device));
+  const int64_t N = Q.N, M = Q.M;
+  cudaStream_t st = o->stream;
+  CKB(cudaMemcpyAsync(Q.starts, starts, (size_t)count * 4, cudaMemcpyHostToDevice, st));
+  if (N > 0) CKB(cudaMemcpyAsync(Q.sigma, sigma, (size_t)count * N * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaMemcpyAsync(Q.dw, dw, (size_t)count * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaMemcpyAsync(Q.dc, dc, (size_t)count * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaMemcpyAsync(Q.rhs, rhs, (size_t)count * M * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaEventRecord(o->ev0, st));
+  const int64_t cap = (int64_t)o->sm_count * 8;
+  int64_t g = ((int64_t)count * M * M + 255) / 256;
+  dnlp_kkt::kkt_zero_kernel<<<(int)(g < cap ? g : cap), 256, 0, st>>>(Q.K, Q.starts, count, M * M);
+  g = (Q.ntgt * count + 255) / 256;
+  dnlp_kkt::kkt_scatter_kernel<<<(int)(g < cap ? g : cap), 256, 0, st>>>(
+      Q.K, Q.Dg, Q.Wd, o->out[4], o->out[5], o->B, Q.ti, Q.tj, Q.sp, Q.src, Q.ntgt, Q.nnzH, Q.starts, count,
+      Q.sigma, Q.dw, Q.dc, N, M);
+  dnlp_kkt::kkt_ldl_kernel<<<count, dnlp_kkt::THREADS, 0, st>>>(Q.K, Q.starts, M, Q.inertia, Q.work, 3 * M);
+  dnlp_kkt::kkt_solve_kernel<<<count, dnlp_kkt::THREADS, 0, st>>>(Q.K, Q.Dg, Q.Wd, Q.starts, M, N, Q.inertia, Q.rhs,
+                                                                  Q.sol, Q.wq, Q.work);
+  o->launches += 4;
+  CKB(cudaPeekAtLastError());
+  CKB(cudaEventRecord(o->ev1, st));
+  CKB(cudaMemcpyAsync(sol, Q.sol, (size_t)count * M * 8, cudaMemcpyDeviceToHost, st));
+  CKB(cudaMemcpyAsync(inertia, Q.inertia, (size_t)count * 3 * 4, cudaMemcpyDeviceToHost, st));
+  CKB(cudaMemcpyAsync(wquad, Q.wq, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
+  CKB(cudaStreamSynchronize(st));
+  float ms = 0.f;
+  CKB(cudaEventElapsedTime(&ms, o->ev0, o->ev1));
+  if (elapsed_ms) *elapsed_ms = ms;
+  return 0;
+}
+
+int dnlp_batch_kkt_matrix(dnlp_batch *o, int32_t start, double *out) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  auto &Q = o->kkt;
+  if (Q.M == 0) { err = "kkt_matrix: call dnlp_batch_kkt_setup first"; return 1; }
+  if (start < 0 || start >= o->B) { err = "kkt_matrix: start id out of range"; return 1; }
+  CKB(cudaSetDevice(o->device));
+  const int64_t M = Q.M;
+  std::vector<double> dg(M);
+  CKB(cudaMemcpyAsync(out, Q.K + (int64_t)start * M * M, (size_t)M * M * 8, cudaMemcpyDeviceToHost, o->stream));
+  CKB(cudaMemcpyAsync(dg.data(), Q.Dg + (int64_t)start * M, (size_t)M * 8, cudaMemcpyDeviceToHost, o->stream));
+  CKB(cudaStreamSynchronize(o->stream));
+  for (int64_t i = 0; i < M; ++i) {         // the strict upper triangle and the saved diagonal are K as assembled
+    out[i * M + i] = dg[i];
+    for (int64_t j = 0; j < i; ++j) out[i * M + j] = out[j * M + i];
+  }
+  return 0;
+}
 
 }  // extern "C"

@@ -101,3 +101,45 @@ class BatchedOracles:
 
     def kernel_launches(self):
         return int(self.dev._L.dnlp_batch_kernel_launches(self.dev.h))
+
+    # ---- batched KKT systems (dnlp_b200/lockstep_ipm.py; include/dnlp_b200.h dnlp_batch_kkt_*) ---------------
+    def kkt_setup(self, slack_rows):
+        """Scatter maps of K = [[W + diag(Sigma) + dw I, A'], [A, -dc I]], A = [J, -P], for the slack rows
+        ``slack_rows`` (the inequality rows, in slack order), and B dense systems in HBM."""
+        sr = np.ascontiguousarray(slack_rows, dtype=np.int32)
+        pats = [np.ascontiguousarray(a, dtype=np.int32) for a in
+                (self.tape.jac_rows, self.tape.jac_cols, self.tape.hess_rows, self.tape.hess_cols)]
+        self.dev.check(self.dev._L.dnlp_batch_kkt_setup(self.dev.h, int(sr.size), sr.ctypes.data_as(_cabi.c_i32p),
+                                                        *[a.ctypes.data_as(_cabi.c_i32p) for a in pats]))
+        self.kkt_N = self.n + int(sr.size)
+        self.kkt_ms = 0.0
+
+    def kkt_solve(self, starts, sigma, dw, dc, rhs):
+        """Assemble, factor (LDL', no pivoting) and solve the systems of the start ids ``starts`` from the JAC and
+        HESS outputs the last device run left in HBM.  ``sigma`` (count, N), ``dw`` / ``dc`` (count,), ``rhs``
+        (count, N + m).  Returns ``(sol, inertia, wquad)``: (count, N + m), (count, 3) int (n+, n-, n0) and
+        dz' W dz; a row whose inertia is not (N, m, 0) or whose refined solution fails the residual test is NaN.
+        ``kkt_ms`` keeps the CUDA-event time of the call's assembly + factorisation + solve."""
+        N, M = self.kkt_N, self.kkt_N + self.m
+        st = np.ascontiguousarray(starts, dtype=np.int32).reshape(-1)
+        cnt = st.size
+        sig = np.ascontiguousarray(sigma, dtype=np.float64).reshape(cnt, N)
+        dw = np.ascontiguousarray(dw, dtype=np.float64).reshape(cnt)
+        dc = np.ascontiguousarray(dc, dtype=np.float64).reshape(cnt)
+        rhs = np.ascontiguousarray(rhs, dtype=np.float64).reshape(cnt, M)
+        sol = np.empty((cnt, M))
+        inertia = np.empty((cnt, 3), dtype=np.int32)
+        wq = np.empty(cnt)
+        ms = C.c_float(0)
+        self.dev.check(self.dev._L.dnlp_batch_kkt_solve(
+            self.dev.h, int(cnt), st.ctypes.data_as(_cabi.c_i32p), _ptr(sig), _ptr(dw), _ptr(dc), _ptr(rhs),
+            _ptr(sol), inertia.ctypes.data_as(_cabi.c_i32p), _ptr(wq), C.byref(ms)))
+        self.kkt_ms = float(ms.value)
+        return sol, inertia, wq
+
+    def kkt_matrix(self, start):
+        """The assembled K of start ``start`` as the last ``kkt_solve`` left it, (N + m, N + m)."""
+        M = self.kkt_N + self.m
+        out = np.empty((M, M))
+        self.dev.check(self.dev._L.dnlp_batch_kkt_matrix(self.dev.h, int(start), _ptr(out)))
+        return out

@@ -199,6 +199,27 @@ int dnlp_batch_profile_groups(dnlp_batch *b, int32_t iters, float *ms_per_group,
                               int32_t max_groups);   /* grouped DMMA GEMM launches, timed with CUDA events */
 int64_t dnlp_batch_kernel_launches(dnlp_batch *b);
 
+/* ---- batched KKT systems of the lock-step interior-point driver (dnlp_b200/lockstep_ipm.py) ----
+ * Per start b, with z = (x, slacks) of length N = n + ns and M = N + m:
+ *   K_b = [[ W_b + diag(Sigma_b) + dw_b I ,  A_b' ],   W_b: the Hessian output HESS (lower-triangle pattern, mirrored,
+ *          [ A_b                          , -dc_b I ]]       duplicates summed in pattern order), zero on the slack block
+ *   A_b = [J_b, -P]: J_b from output JAC, column n + s of P is a 1 in constraint row slack_rows[s].
+ * dnlp_batch_kkt_setup builds the scatter maps from the patterns (host arrays) and allocates B dense M x M systems;
+ * it fails with a message naming B*M^2*8 bytes when they do not fit.  dnlp_batch_kkt_solve assembles K for `count`
+ * distinct start ids from the HESS and JAC outputs the last run left in HBM, factors it as LDL' without pivoting
+ * (order [x / slack block, constraint block]) and returns per start the inertia (n+, n-, n0) from the signs of D
+ * (a pivot d_j with |d_j| <= 1e-11 (|K_jj| + sum_k L_jk^2 |d_k|) counts as zero).  For a start whose inertia is (N, m, 0) it solves K sol = rhs,
+ * refines once against K and returns the solution and dz' W dz (dz = sol[:N]); the solution row and wquad are NaN
+ * when the inertia differs, the result is not finite, or its normwise backward error exceeds 1e-8.
+ * Inputs and outputs are start-major: sigma[c*N + i], rhs / sol[c*M + i], inertia[3c + k].  *elapsed_ms: CUDA-event
+ * time of assembly + factorisation + solve.  dnlp_batch_kkt_matrix copies the assembled K of one start (M x M). */
+int dnlp_batch_kkt_setup(dnlp_batch *b, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                         const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols);
+int dnlp_batch_kkt_solve(dnlp_batch *b, int32_t count, const int32_t *starts, const double *sigma, const double *dw,
+                         const double *dc, const double *rhs, double *sol, int32_t *inertia, double *wquad,
+                         float *elapsed_ms);
+int dnlp_batch_kkt_matrix(dnlp_batch *b, int32_t start, double *out);
+
 /* ---- row-sharded evaluation across the GPUs of one node (BASELINE config 3; SURVEY.md 8e) ----
  * One process per GPU.  The reference has no counterpart (it is single-process NumPy); the surface
  * mirrors the callbacks above, evaluated collectively: every rank runs the local tape of its rows,
