@@ -32,6 +32,7 @@ struct BInstr {
   int gemm_group = -1;               // index into dnlp_batch::groups when this GEMV runs in a grouped launch
   dnlp::GemmDesc *one_desc = nullptr;   // device descriptor for launching this GEMV on its own
   int32_t *smallk_slots = nullptr;   // device: the K slots every row combines (tall-skinny GEMM path)
+  std::string kname;                 // kernel variant the last launch of this instruction ran (dnlp_batch_instr_kernel)
 };
 }  // namespace
 
@@ -92,7 +93,7 @@ struct dnlp_batch {
   double *split_scratch = nullptr;         // partial sums of the term-split long-row kernel
   unsigned int *split_tickets = nullptr;
   int64_t split_scratch_len = 0, split_ticket_len = 0;
-  int launch(const BInstr &I);
+  int launch(BInstr &I);
   int run_program(int p);
   int run_union(int32_t prog_mask);
   int issue_union(int32_t prog_mask);
@@ -109,10 +110,10 @@ void launch_belem_t(const dnlp_batch *o, const dnlp_instr_desc &d, int grid) {
   belem_kernel<F, Bn><<<grid, 256, 0, o->stream>>>(o->V, d.a_off, d.a_stride, d.b_off, d.b_stride, d.dst_off,
                                                   d.count, d.param, o->B, d.dst_stride > 0 ? d.dst_stride : 1, d.post_scale);
 }
-bool launch_belem(const dnlp_batch *o, const dnlp_instr_desc &d, int grid) {
+bool launch_belem(const dnlp_batch *o, const dnlp_instr_desc &d, int grid, std::string &kname) {
   switch (d.fcode) {
-#define U(F) case F: launch_belem_t<F, false>(o, d, grid); return true;
-#define Bn(F) case F: launch_belem_t<F, true>(o, d, grid); return true;
+#define U(F) case F: launch_belem_t<F, false>(o, d, grid); kname = "belem_kernel<" + std::to_string(F) + ", 0>"; return true;
+#define Bn(F) case F: launch_belem_t<F, true>(o, d, grid); kname = "belem_kernel<" + std::to_string(F) + ", 1>"; return true;
     U(F_EXP) U(F_LOG) U(F_ENTR) U(F_NEG_LOG_M1) U(F_RECIP) U(F_NEG_RECIP) U(F_NEG_RECIP_SQ)
     U(F_LOGISTIC) U(F_LOGISTIC_D1) U(F_LOGISTIC_D2) U(F_POW)
     U(F_SIN) U(F_COS) U(F_NEG_SIN) U(F_NEG_COS) U(F_TAN) U(F_TAN_D1) U(F_TAN_D2)
@@ -127,13 +128,13 @@ bool launch_belem(const dnlp_batch *o, const dnlp_instr_desc &d, int grid) {
 }
 }  // namespace
 
-int dnlp_batch::launch(const BInstr &I) {
+int dnlp_batch::launch(BInstr &I) {
   const dnlp_instr_desc &d = I.d;
   if (d.count <= 0) return 0;
   double *dst = (d.dst_space == DNLP_DST_V) ? V + d.dst_off * B : out[d.dst_space] + d.dst_off * B;
   switch (d.kind) {
     case DNLP_ELEM:
-      if (!launch_belem(this, d, grid_for(d.count * B))) { err = "unknown elementwise function code"; return 1; }
+      if (!launch_belem(this, d, grid_for(d.count * B), I.kname)) { err = "unknown elementwise function code"; return 1; }
       break;
     case DNLP_POLY: {
       if (I.smallk_slots) {
@@ -149,7 +150,8 @@ int dnlp_batch::launch(const BInstr &I) {
         const int64_t blocks = ((d.count + rows_per_block - 1) / rows_per_block) * bchunks;
 #define SKN(Lc, Nb) bsmallk_kernel<Lc, Nb><<<(int)blocks, threads, 0, stream>>>(                      \
             V, dst, d.coef, I.smallk_slots, d.pos, d.count, d.accumulate, B, rows_per_block)
-#define SK(Lc) case Lc: if (nb == 4) SKN(Lc, 4); else if (nb == 2) SKN(Lc, 2); else SKN(Lc, 1); break;
+#define SK(Lc) case Lc: if (nb == 4) SKN(Lc, 4); else if (nb == 2) SKN(Lc, 2); else SKN(Lc, 1); \
+          I.kname = "bsmallk_kernel<" #Lc ", " + std::to_string(nb) + ">"; break;
         switch (d.row_len) {
           SK(2) SK(3) SK(4) SK(5) SK(6) SK(7) SK(8) SK(9) SK(10) SK(11) SK(12) SK(13) SK(14) SK(15) SK(16)
           default: err = "small-K kernel: unsupported row length"; return 1;
@@ -170,6 +172,7 @@ int dnlp_batch::launch(const BInstr &I) {
             bpoly_long_split_kernel<true, 8><<<(int)(blocks * KS), 256, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B, KS, split_scratch, split_tickets);
           else
             bpoly_long_split_kernel<false, 8><<<(int)(blocks * KS), 256, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B, KS, split_scratch, split_tickets);
+          I.kname = std::string("bpoly_long_split_kernel<") + (I.has_f2 ? "1" : "0") + ", 8>";
           break;
         }
         // few (row, start-chunk) pairs: 16 warps split the terms; enough of them to fill the machine: 8
@@ -178,6 +181,7 @@ int dnlp_batch::launch(const BInstr &I) {
             bpoly_long_kernel<true, 16><<<(int)blocks, 512, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
           else
             bpoly_long_kernel<false, 16><<<(int)blocks, 512, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
+          I.kname = std::string("bpoly_long_kernel<") + (I.has_f2 ? "1" : "0") + ", 16>";
         } else {
           const int64_t cap = (int64_t)sm_count * 8;
           const int grid = (int)(blocks < cap ? blocks : cap);
@@ -185,6 +189,7 @@ int dnlp_batch::launch(const BInstr &I) {
             bpoly_long_kernel<true, 8><<<grid, 256, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
           else
             bpoly_long_kernel<false, 8><<<grid, 256, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
+          I.kname = std::string("bpoly_long_kernel<") + (I.has_f2 ? "1" : "0") + ", 8>";
         }
         break;
       }
@@ -196,6 +201,7 @@ int dnlp_batch::launch(const BInstr &I) {
         bpoly_kernel<true><<<grid, threads, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
       else
         bpoly_kernel<false><<<grid, threads, 0, stream>>>(V, dst, d.ptr, d.row_len, d.coef, d.f1, d.f2, d.pos, d.count, d.accumulate, B);
+      I.kname = std::string("bpoly_kernel<") + (I.has_f2 ? "1" : "0") + ">";
       break;
     }
     case DNLP_GEMV: {
@@ -206,10 +212,12 @@ int dnlp_batch::launch(const BInstr &I) {
         bgemm_dmma_kernel<true><<<tiles < cap ? tiles : cap, 128, BGEMM_SMEM, stream>>>(I.one_desc, 1, (int)d.count, B, (int)d.ncols);
       else
         bgemm_dmma_kernel<false><<<tiles < cap ? tiles : cap, 128, BGEMM_SMEM, stream>>>(I.one_desc, 1, (int)d.count, B, (int)d.ncols);
+      I.kname = dmma_k8 ? "bgemm_dmma_kernel<1>" : "bgemm_dmma_kernel<0>";
       break;
     }
     case DNLP_SCALE:
       bscale_kernel<<<grid_for(d.count * B), 256, 0, stream>>>(V, d.s_slot, d.coef, dst, d.pos, d.count, d.accumulate, B);
+      I.kname = "bscale_kernel";
       break;
     default:
       err = "unknown instruction kind";
@@ -270,6 +278,7 @@ int dnlp_batch::issue_union(int32_t prog_mask) {
       else
         bgemm_dmma_kernel<false><<<(int)(tiles < cap ? tiles : cap), 128, BGEMM_SMEM, stream>>>(
             G.descs, (int)G.members.size(), (int)G.M, B, (int)G.K);
+      for (int32_t mid : G.members) instrs[mid].kname = dmma_k8 ? "bgemm_dmma_kernel<1>" : "bgemm_dmma_kernel<0>";
       ++launches;
       cudaError_t e = cudaPeekAtLastError();
       if (e != cudaSuccess) { err = std::string("kernel launch failed: ") + cudaGetErrorString(e); return 1; }
@@ -576,6 +585,12 @@ int dnlp_batch_profile_groups(dnlp_batch *o, int32_t iters, float *ms_per_group,
 }
 
 int64_t dnlp_batch_kernel_launches(dnlp_batch *o) { return o ? o->launches : -1; }
+
+const char *dnlp_batch_instr_kernel(dnlp_batch *o, int32_t instr) {
+  if (!o) return "";
+  if (instr < 0 || (size_t)instr >= o->instrs.size()) return "";
+  return o->instrs[instr].kname.c_str();
+}
 
 int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
                          const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols) {

@@ -102,6 +102,11 @@ class BatchedOracles:
     def kernel_launches(self):
         return int(self.dev._L.dnlp_batch_kernel_launches(self.dev.h))
 
+    def instr_kernel(self, instr):
+        """Name of the kernel variant that ran instruction ``instr`` (template arguments included, e.g.
+        ``bsmallk_kernel<9, 2>``); "" for an instruction no evaluation has launched yet."""
+        return self.dev._L.dnlp_batch_instr_kernel(self.dev.h, int(instr)).decode()
+
     # ---- batched KKT systems (dnlp_b200/lockstep_ipm.py; include/dnlp_b200.h dnlp_batch_kkt_*) ---------------
     def kkt_setup(self, slack_rows):
         """Scatter maps of K = [[W + diag(Sigma) + dw I, A'], [A, -dc I]], A = [J, -P], for the slack rows

@@ -198,6 +198,8 @@ int dnlp_batch_profile_instrs(dnlp_batch *b, int32_t prog, int32_t iters, float 
 int dnlp_batch_profile_groups(dnlp_batch *b, int32_t iters, float *ms_per_group, double *flops_per_group,
                               int32_t max_groups);   /* grouped DMMA GEMM launches, timed with CUDA events */
 int64_t dnlp_batch_kernel_launches(dnlp_batch *b);
+const char *dnlp_batch_instr_kernel(dnlp_batch *b, int32_t instr);   /* kernel variant of an executed instruction, e.g.
+                                                                          "bsmallk_kernel<9, 2>"; "" if never run */
 
 /* ---- batched KKT systems of the lock-step interior-point driver (dnlp_b200/lockstep_ipm.py) ----
  * Per start b, with z = (x, slacks) of length N = n + ns and M = N + m:

@@ -59,6 +59,9 @@ def test_null_handle_is_an_error_not_a_crash():
     assert L.dnlp_upload_point(None, p, p, 1.0) != 0
     assert L.dnlp_batch_upload(None, p, p, p) != 0
     assert L.dnlp_kernel_launches(None) == -1
+    assert L.dnlp_batch_kernel_launches(None) == -1
+    assert L.dnlp_instr_kernel(None, 0) == b""
+    assert L.dnlp_batch_instr_kernel(None, 0) == b""
     assert b"NULL" in L.dnlp_last_error(None)
     # the sharded oracle's host-side entry points (shared-host delivery, worker loop) as well
     import ctypes as C
