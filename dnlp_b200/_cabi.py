@@ -56,6 +56,7 @@ EXPORTS = [
     "dnlp_batch_create", "dnlp_batch_destroy", "dnlp_batch_last_error", "dnlp_batch_eval", "dnlp_batch_upload",
     "dnlp_batch_run_device", "dnlp_batch_read_output", "dnlp_batch_profile_instrs", "dnlp_batch_kernel_launches", "dnlp_batch_profile_groups", "dnlp_batch_instr_kernel",
     "dnlp_batch_kkt_setup", "dnlp_batch_kkt_solve", "dnlp_batch_kkt_matrix",
+    "dnlp_batch_kkt_setup_qn", "dnlp_batch_qn_update", "dnlp_batch_qn_matrix",
     "dnlp_comm_unique_id", "dnlp_comm_create", "dnlp_comm_destroy", "dnlp_comm_last_error", "dnlp_comm_has_nccl",
     "dnlp_comm_ipc_handle", "dnlp_comm_open_peers", "dnlp_comm_allreduce_host",
     "dnlp_shard_create", "dnlp_shard_destroy", "dnlp_shard_last_error", "dnlp_shard_set_output",
@@ -137,6 +138,9 @@ def lib():
     L.dnlp_batch_kkt_setup.argtypes = [vp, C.c_int64] + [c_i32p] * 5
     L.dnlp_batch_kkt_solve.argtypes = [vp, C.c_int32, c_i32p] + [c_f64p] * 5 + [c_i32p, c_f64p, c_f32p]
     L.dnlp_batch_kkt_matrix.argtypes = [vp, C.c_int32, c_f64p]
+    L.dnlp_batch_kkt_setup_qn.argtypes = [vp, C.c_int64] + [c_i32p] * 3
+    L.dnlp_batch_qn_update.argtypes = [vp, C.c_int32, c_i32p, c_f64p, c_f64p, c_i32p, c_f32p]
+    L.dnlp_batch_qn_matrix.argtypes = [vp, C.c_int32, c_f64p]
     cp = C.c_char_p
     L.dnlp_comm_unique_id.argtypes = [cp]
     L.dnlp_comm_create.argtypes = [cp, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]

@@ -83,25 +83,31 @@ def _equality_only(problem_ir):
     return not any(finite) and not two_sided
 
 
-def best_of_lockstep(problem_ir, X0, device=0, evaluator=None, kkt=None, tol=None, max_iter=None):
+def best_of_lockstep(problem_ir, X0, device=0, evaluator=None, kkt=None, tol=None, max_iter=None,
+                     hessian_approximation="exact"):
     """All starts ``X0`` (B, n) of one smooth problem in lock step on the GPU; ``evaluator`` replaces
     ``BatchedOracles`` (CPU tests).  Equality-constrained problems without bounds take ``lockstep_newton_kkt``
     (defaults tol 1e-12, 60 iterations), every other problem ``lockstep_ipm`` (tol 1e-8, 500 iterations) with the KKT
-    backend ``kkt`` (default: ``DeviceKKT`` on the evaluator).  Adds ``all_objs`` and ``best`` (index of the smallest
-    objective among the converged starts) to the solver's result."""
+    backend ``kkt`` (default: ``DeviceKKT`` on the evaluator).  ``hessian_approximation="limited-memory"`` (IPOPT's
+    option name) sends every problem to ``lockstep_ipm`` with a damped-BFGS Hessian per start: the Newton-KKT
+    iteration needs the exact Hessian.  Adds ``all_objs`` and ``best`` (index of the smallest objective among the
+    converged starts) to the solver's result."""
+    from .lockstep_ipm import check_hessian_approximation
+    qn = check_hessian_approximation(hessian_approximation)
     own = evaluator is None
     if own:
         from .multistart import BatchedOracles
         evaluator = BatchedOracles(problem_ir, len(X0), device=device)
     try:
-        if _equality_only(problem_ir):
+        if _equality_only(problem_ir) and not qn:
             out = lockstep_newton_kkt(evaluator, X0, tol=1e-12 if tol is None else tol,
                                       max_iter=60 if max_iter is None else max_iter)
         else:
             from .lockstep_ipm import DeviceKKT, lockstep_ipm
-            out = lockstep_ipm(evaluator, DeviceKKT(evaluator) if kkt is None else kkt, X0, lb=problem_ir.lb,
-                               ub=problem_ir.ub, cl=problem_ir.cl, cu=problem_ir.cu, tol=1e-8 if tol is None else tol,
-                               max_iter=500 if max_iter is None else max_iter)
+            out = lockstep_ipm(evaluator, DeviceKKT(evaluator, quasi_newton=qn) if kkt is None else kkt, X0,
+                               lb=problem_ir.lb, ub=problem_ir.ub, cl=problem_ir.cl, cu=problem_ir.cu,
+                               tol=1e-8 if tol is None else tol, max_iter=500 if max_iter is None else max_iter,
+                               hessian_approximation=hessian_approximation)
             out["converged"] = out["status"] == 0
     finally:
         if own:
@@ -127,7 +133,9 @@ def solve_best_of(prob, best_of, solver="lockstep", device=0, evaluator_factory=
     ``solver``: "lockstep" (all starts at once on the GPU: the Newton-KKT iteration for equality-constrained problems
     without bounds, the lock-step interior-point method for every other problem) or "ipopt" (per-start
     ``solve_via_data`` on the shared resident oracle; needs cyipopt).  ``evaluator_factory(problem_ir, B)`` and
-    ``kkt_factory(evaluator)`` replace ``BatchedOracles`` and the device KKT backend (CPU tests).
+    ``kkt_factory(evaluator)`` replace ``BatchedOracles`` and the device KKT backend (CPU tests); with
+    ``hessian_approximation="limited-memory"`` in ``solver_opts`` the latter is called as
+    ``kkt_factory(evaluator, quasi_newton=True)``.
 
     ``faithful`` (default): the reference's loop ranks the starts by ``self.objective.value`` with ``<`` whatever the
     sense (problem.py:1262-1268), so for a Maximize problem it keeps the start with the SMALLEST objective, and it
@@ -165,7 +173,11 @@ def solve_best_of(prob, best_of, solver="lockstep", device=0, evaluator_factory=
     else:
         pir = data_to_ir(data)
         ev = evaluator_factory(pir, best_of) if evaluator_factory is not None else None
-        kkt = kkt_factory(ev) if (kkt_factory is not None and ev is not None) else None
+        kkt = None
+        if kkt_factory is not None and ev is not None:
+            from .lockstep_ipm import check_hessian_approximation
+            qn = check_hessian_approximation(solver_opts.get("hessian_approximation", "exact"))
+            kkt = kkt_factory(ev, quasi_newton=True) if qn else kkt_factory(ev)
         out = best_of_lockstep(pir, np.stack(starts), device=device, evaluator=ev, kkt=kkt, **solver_opts)
         objs = out["all_objs"]
         best = _pick(np.asarray(objs), maximize, faithful)

@@ -3,6 +3,7 @@
 #include "../../include/dnlp_b200.h"
 #include "dnlp_batch_kernels.cuh"
 #include "dnlp_batch_kkt.cuh"
+#include "dnlp_batch_qn.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -62,6 +63,12 @@ struct dnlp_batch {
     double *K = nullptr, *Dg = nullptr, *Wd = nullptr, *work = nullptr;
     double *sigma = nullptr, *dw = nullptr, *dc = nullptr, *rhs = nullptr, *sol = nullptr, *wq = nullptr;
     int32_t *starts = nullptr, *inertia = nullptr;
+    // quasi-Newton mode (dnlp_batch_kkt_setup_qn): W_b packed (n(n+1)/2 x B, batch fastest) takes HESS's place as the
+    // source of the x-block, ids < nnzH of the scatter map index it; update scratch is n x B, start fastest
+    bool qn = false;
+    double *Wq = nullptr, *qS = nullptr, *qY = nullptr, *qSt = nullptr, *qYt = nullptr, *qBs = nullptr, *qR = nullptr;
+    double *qcoef = nullptr;
+    int32_t *qstarts = nullptr, *qapplied = nullptr;
     std::vector<void *> owned;
   } kkt;
   void kkt_free() {
@@ -592,15 +599,25 @@ const char *dnlp_batch_instr_kernel(dnlp_batch *o, int32_t instr) {
   return o->instrs[instr].kname.c_str();
 }
 
-int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
-                         const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols) {
-  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+// the scatter map and the workspaces of both modes.  Exact mode: the x-block's sources are the HESS pattern
+// (hess_rows / hess_cols).  Quasi-Newton mode (hess_rows == nullptr): they are the packed lower triangle of W_b,
+// source id p = i (i + 1) / 2 + j, and W_b := I.
+static int kkt_setup_impl(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                          const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols, bool qn) {
   std::string &err = o->err;
   CKB(cudaSetDevice(o->device));
   CKB(cudaStreamSynchronize(o->stream));
   o->kkt_free();
-  const int64_t n = o->n, m = o->m, nnzJ = o->out_len[4], nnzH = o->out_len[5];
+  const int64_t n = o->n, m = o->m, nnzJ = o->out_len[4];
+  const int64_t nnzH = qn ? n * (n + 1) / 2 : o->out_len[5];
   if (ns < 0 || ns > m) { err = "kkt_setup: the number of slack rows must lie in [0, m]"; return 1; }
+  if (qn && nnzH + nnzJ > (int64_t)INT32_MAX) {
+    char buf[256];
+    snprintf(buf, sizeof buf, "kkt_setup_qn: n = %lld gives n(n+1)/2 = %lld packed entries, which with %lld Jacobian "
+             "entries exceed the int32 index range of the scatter map", (long long)n, (long long)nnzH, (long long)nnzJ);
+    err = buf;
+    return 1;
+  }
   const int64_t N = n + ns, M = N + m, B = o->B;
   // the scatter map: every lower-triangle target (i, j) of K with its sources in pattern order
   std::map<int64_t, std::vector<int32_t>> tgt;
@@ -611,10 +628,15 @@ int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, c
     if (r < 0 || r >= m || seen[r]) { err = "kkt_setup: slack rows must be distinct constraint rows"; return 1; }
     seen[r] = 1;
   }
-  for (int64_t k = 0; k < nnzH; ++k) {
-    const int64_t r = hess_rows[k], c = hess_cols[k];
-    if (r < 0 || r >= n || c < 0 || c >= n) { err = "kkt_setup: Hessian pattern entry out of range"; return 1; }
-    tgt[std::max(r, c) * M + std::min(r, c)].push_back((int32_t)k);
+  if (qn) {
+    for (int64_t i = 0, p = 0; i < n; ++i)
+      for (int64_t j = 0; j <= i; ++j, ++p) tgt[i * M + j].push_back((int32_t)p);
+  } else {
+    for (int64_t k = 0; k < nnzH; ++k) {
+      const int64_t r = hess_rows[k], c = hess_cols[k];
+      if (r < 0 || r >= n || c < 0 || c >= n) { err = "kkt_setup: Hessian pattern entry out of range"; return 1; }
+      tgt[std::max(r, c) * M + std::min(r, c)].push_back((int32_t)k);
+    }
   }
   for (int64_t k = 0; k < nnzJ; ++k) {
     const int64_t r = jac_rows[k], c = jac_cols[k];
@@ -629,16 +651,24 @@ int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, c
     src.insert(src.end(), kv.second.begin(), kv.second.end());
     sp.push_back((int32_t)src.size());
   }
-  // refuse what does not fit: the B dense systems dominate
+  // refuse what does not fit: the B dense systems (and in quasi-Newton mode the B packed W) dominate
   const double kbytes = (double)B * (double)M * (double)M * 8.0;
-  const double vbytes = (double)B * (double)(9 * M + 2 * N + 4) * 8.0 + (double)(3 * ti.size() + src.size() + 1) * 4.0;
+  const double wbytes = qn ? (double)B * (double)nnzH * 8.0 : 0.0;
+  const double vbytes = (double)B * (double)(9 * M + 2 * N + 4 + (qn ? 6 * n + 3 : 0)) * 8.0 +
+                        (double)(3 * ti.size() + src.size() + 1) * 4.0;
   size_t free_b = 0, total_b = 0;
   CKB(cudaMemGetInfo(&free_b, &total_b));
-  if (kbytes + vbytes > 0.95 * (double)free_b) {
-    char buf[320];
-    snprintf(buf, sizeof buf, "kkt_setup: the dense KKT systems need B*(N+m)^2*8 = %lld*%lld^2*8 = %.3e bytes "
-             "(+%.3e for vectors) but the device has %.3e bytes free; use fewer starts per batch",
-             (long long)B, (long long)M, kbytes, vbytes, (double)free_b);
+  if (kbytes + wbytes + vbytes > 0.95 * (double)free_b) {
+    char buf[400];
+    if (qn)
+      snprintf(buf, sizeof buf, "kkt_setup_qn: the dense KKT systems need B*(N+m)^2*8 = %lld*%lld^2*8 = %.3e bytes and "
+               "the quasi-Newton matrices B*n(n+1)/2*8 = %lld*%lld*8 = %.3e bytes (+%.3e for vectors) but the device "
+               "has %.3e bytes free; use fewer starts per batch", (long long)B, (long long)M, kbytes, (long long)B,
+               (long long)nnzH, wbytes, vbytes, (double)free_b);
+    else
+      snprintf(buf, sizeof buf, "kkt_setup: the dense KKT systems need B*(N+m)^2*8 = %lld*%lld^2*8 = %.3e bytes "
+               "(+%.3e for vectors) but the device has %.3e bytes free; use fewer starts per batch",
+               (long long)B, (long long)M, kbytes, vbytes, (double)free_b);
     err = buf;
     return 1;
   }
@@ -664,7 +694,97 @@ int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, c
     o->kkt_free();
     return 1;
   }
+  if (qn) {
+    const size_t vec = (size_t)B * n * 8;
+    if (alloc((size_t)B * nnzH * 8, (void **)&Q.Wq) || alloc(vec, (void **)&Q.qS) || alloc(vec, (void **)&Q.qY) ||
+        alloc(vec, (void **)&Q.qSt) || alloc(vec, (void **)&Q.qYt) || alloc(vec, (void **)&Q.qBs) ||
+        alloc(vec, (void **)&Q.qR) || alloc((size_t)B * 2 * 8, (void **)&Q.qcoef) ||
+        alloc((size_t)B * 4, (void **)&Q.qstarts) || alloc((size_t)B * 4, (void **)&Q.qapplied)) {
+      o->kkt_free();
+      return 1;
+    }
+    Q.qn = true;
+    if (nnzH > 0) {
+      dnlp_qn::qn_identity_kernel<<<o->grid_for(nnzH * B), 256, 0, o->stream>>>(Q.Wq, nnzH, o->B);
+      ++o->launches;
+    }
+  }
+  cudaError_t e = cudaPeekAtLastError();
+  if (e == cudaSuccess) e = cudaStreamSynchronize(o->stream);
+  if (e != cudaSuccess) {
+    o->kkt_free();
+    err = std::string("kkt_setup: ") + cudaGetErrorString(e);
+    return 1;
+  }
+  return 0;
+}
+
+int dnlp_batch_kkt_setup(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                         const int32_t *jac_cols, const int32_t *hess_rows, const int32_t *hess_cols) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  return kkt_setup_impl(o, ns, slack_rows, jac_rows, jac_cols, hess_rows, hess_cols, false);
+}
+
+int dnlp_batch_kkt_setup_qn(dnlp_batch *o, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                            const int32_t *jac_cols) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  return kkt_setup_impl(o, ns, slack_rows, jac_rows, jac_cols, nullptr, nullptr, true);
+}
+
+int dnlp_batch_qn_update(dnlp_batch *o, int32_t count, const int32_t *starts, const double *S, const double *Y,
+                         int32_t *applied, float *elapsed_ms) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  auto &Q = o->kkt;
+  if (!Q.qn) { err = "qn_update: call dnlp_batch_kkt_setup_qn first"; return 1; }
+  if (count < 0 || count > o->B) { err = "qn_update: count must lie in [0, batch]"; return 1; }
+  if (elapsed_ms) *elapsed_ms = 0.f;
+  std::vector<char> seen(o->B, 0);
+  for (int c = 0; c < count; ++c) {
+    if (starts[c] < 0 || starts[c] >= o->B || seen[starts[c]]) { err = "qn_update: start ids must be distinct and in [0, batch)"; return 1; }
+    seen[starts[c]] = 1;
+  }
+  const int64_t n = o->n, np = n * (n + 1) / 2;
+  if (count == 0 || n == 0) {
+    for (int c = 0; c < count; ++c) applied[c] = 0;
+    return 0;
+  }
+  CKB(cudaSetDevice(o->device));
+  cudaStream_t st = o->stream;
+  CKB(cudaMemcpyAsync(Q.qstarts, starts, (size_t)count * 4, cudaMemcpyHostToDevice, st));
+  CKB(cudaMemcpyAsync(Q.qS, S, (size_t)count * n * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaMemcpyAsync(Q.qY, Y, (size_t)count * n * 8, cudaMemcpyHostToDevice, st));
+  CKB(cudaEventRecord(o->ev0, st));
+  dnlp_qn::qn_transpose_kernel<<<o->grid_for(n * count), 256, 0, st>>>(Q.qS, Q.qY, Q.qSt, Q.qYt, n, count);
+  dnlp_qn::qn_gemv_kernel<<<o->grid_for(n * count), 256, 0, st>>>(Q.Wq, o->B, Q.qstarts, count, Q.qSt, Q.qBs, n);
+  dnlp_qn::qn_coef_kernel<<<(count + 127) / 128, 128, 0, st>>>(Q.qSt, Q.qYt, Q.qBs, Q.qR, Q.qcoef, Q.qapplied, n, count);
+  dnlp_qn::qn_rank2_kernel<<<o->grid_for(np * count), 256, 0, st>>>(Q.Wq, o->B, Q.qstarts, count, Q.qBs, Q.qR,
+                                                                     Q.qcoef, Q.qapplied, np);
+  o->launches += 4;
+  CKB(cudaPeekAtLastError());
+  CKB(cudaEventRecord(o->ev1, st));
+  CKB(cudaMemcpyAsync(applied, Q.qapplied, (size_t)count * 4, cudaMemcpyDeviceToHost, st));
+  CKB(cudaStreamSynchronize(st));
+  float ms = 0.f;
+  CKB(cudaEventElapsedTime(&ms, o->ev0, o->ev1));
+  if (elapsed_ms) *elapsed_ms = ms;
+  return 0;
+}
+
+int dnlp_batch_qn_matrix(dnlp_batch *o, int32_t start, double *out) {
+  if (o == nullptr) { g_batch_create_error = "batch handle is NULL (closed or never created)"; return 1; }
+  std::string &err = o->err;
+  auto &Q = o->kkt;
+  if (!Q.qn) { err = "qn_matrix: call dnlp_batch_kkt_setup_qn first"; return 1; }
+  if (start < 0 || start >= o->B) { err = "qn_matrix: start id out of range"; return 1; }
+  CKB(cudaSetDevice(o->device));
+  const int64_t n = o->n, np = n * (n + 1) / 2;
+  std::vector<double> w((size_t)np);                  // column `start` of the np x B packed array
+  CKB(cudaMemcpy2DAsync(w.data(), 8, Q.Wq + start, (size_t)o->B * 8, 8, (size_t)np, cudaMemcpyDeviceToHost,
+                        o->stream));
   CKB(cudaStreamSynchronize(o->stream));
+  for (int64_t i = 0, p = 0; i < n; ++i)
+    for (int64_t j = 0; j <= i; ++j, ++p) out[i * n + j] = out[j * n + i] = w[p];
   return 0;
 }
 
@@ -696,7 +816,7 @@ int dnlp_batch_kkt_solve(dnlp_batch *o, int32_t count, const int32_t *starts, co
   dnlp_kkt::kkt_zero_kernel<<<(int)(g < cap ? g : cap), 256, 0, st>>>(Q.K, Q.starts, count, M * M);
   g = (Q.ntgt * count + 255) / 256;
   dnlp_kkt::kkt_scatter_kernel<<<(int)(g < cap ? g : cap), 256, 0, st>>>(
-      Q.K, Q.Dg, Q.Wd, o->out[4], o->out[5], o->B, Q.ti, Q.tj, Q.sp, Q.src, Q.ntgt, Q.nnzH, Q.starts, count,
+      Q.K, Q.Dg, Q.Wd, o->out[4], Q.qn ? Q.Wq : o->out[5], o->B, Q.ti, Q.tj, Q.sp, Q.src, Q.ntgt, Q.nnzH, Q.starts, count,
       Q.sigma, Q.dw, Q.dc, N, M);
   dnlp_kkt::kkt_ldl_kernel<<<count, dnlp_kkt::THREADS, 0, st>>>(Q.K, Q.starts, M, Q.inertia, Q.work, 3 * M);
   dnlp_kkt::kkt_solve_kernel<<<count, dnlp_kkt::THREADS, 0, st>>>(Q.K, Q.Dg, Q.Wd, Q.starts, M, N, Q.inertia, Q.rhs,

@@ -34,7 +34,8 @@ __global__ void kkt_zero_kernel(double *K, const int32_t *starts, int count, int
 
 // One thread per (target entry, selected start), start fastest: the output reads (len x B, batch fastest) coalesce.
 // Target t sums its sources in the fixed order of src[sp[t] .. sp[t+1]): id < nnzH -> HESS[id], id >= nnzH ->
-// JAC[id - nnzH], id == -1 -> the constant -1 of the slack column.  A diagonal target of the x / slack block then adds
+// JAC[id - nnzH], id == -1 -> the constant -1 of the slack column.  In quasi-Newton mode `hess` is the packed W of
+// dnlp_batch_qn.cuh (same batch-fastest layout, nnzH = n(n+1)/2) and each x-block target has its one packed entry.  A diagonal target of the x / slack block then adds
 // Sigma and dw, one of the constraint block is -dc:  K_ii = (W_ii + Sigma_i) + dw.
 __global__ void kkt_scatter_kernel(double *K, double *Dg, double *Wd, const double *__restrict__ jac,
                                    const double *__restrict__ hess, int B, const int32_t *__restrict__ ti,

@@ -16,7 +16,15 @@ One outer iteration:
 
 The KKT backend is a constructor argument.  ``DeviceKKT`` keeps the Hessian and Jacobian in HBM and factors the
 systems there (csrc/dnlp_batch_kkt.cuh, LDL' without pivoting); the test-suite passes a NumPy implementation of the
-same factorisation.  Not covered: the quasi-Newton branch (no Hessian) and the ``intermediate`` callback.
+same factorisation.
+
+``hessian_approximation="limited-memory"`` is the stand-in's quasi-Newton branch: W is a dense damped-BFGS matrix per
+start, W_0 = I, updated after every accepted step (except the one that ends a start on the stall rule) with
+s = x_new - x_old and y = (grad f + J'lam)(x_new) - (grad f + J'lam)(x_old), both with the new lam.  The update runs
+at the top of the next outer iteration on the starts accepted in the previous one that are still active, from that
+iteration's f / grad f / g / J evaluation (no extra evaluation); step 2 then evaluates only J, the Hessian is never
+asked for.  With ``DeviceKKT(ev, quasi_newton=True)`` the matrices live in HBM and the update runs there
+(csrc/dnlp_batch_qn.cuh).  Not covered: IPOPT's compact L-BFGS and the ``intermediate`` callback.
 """
 import time
 
@@ -35,19 +43,32 @@ STATUS_MSG = {0: b"Algorithm terminated successfully at a locally optimal point"
 
 class DeviceKKT:
     """KKT backend on ``BatchedOracles``: the Hessian and Jacobian never leave HBM; the B dense systems are assembled,
-    factored and solved there (``BatchedOracles.kkt_solve``)."""
+    factored and solved there (``BatchedOracles.kkt_solve``).  With ``quasi_newton`` the Hessian is replaced by one
+    damped-BFGS matrix per start, kept and updated in HBM (``BatchedOracles.qn_update``)."""
 
-    def __init__(self, ev):
+    def __init__(self, ev, quasi_newton=False):
         self.ev = ev
-        self.device_ms = 0.0          # CUDA-event time of assembly + factorisation + solve, summed over calls
+        self.quasi_newton = bool(quasi_newton)
+        self.device_ms = 0.0          # CUDA-event time of assembly + factorisation + solve (+ QN update), summed
+        self.qn_ms = 0.0              # CUDA-event time of the quasi-Newton updates alone
+        self.qn_calls = self.qn_starts = 0
 
     def setup(self, slack_rows):
-        self.ev.kkt_setup(slack_rows)
+        self.ev.kkt_setup(slack_rows, quasi_newton=self.quasi_newton)
 
     def load(self, X, LAM):
-        """The Jacobian and the Hessian of the Lagrangian (sigma = 1) of every start at (X, LAM), on the device."""
+        """The Jacobian and (exact mode) the Hessian of the Lagrangian (sigma = 1) of every start at (X, LAM), on the
+        device."""
         self.ev.upload(X, LAM, np.ones(X.shape[0]))
-        self.ev.run_device(("jac", "hess"))
+        self.ev.run_device(("jac",) if self.quasi_newton else ("jac", "hess"))
+
+    def update(self, starts, S, Y):
+        applied = self.ev.qn_update(starts, S, Y)
+        self.qn_ms += self.ev.qn_ms
+        self.device_ms += self.ev.qn_ms
+        self.qn_calls += 1
+        self.qn_starts += len(starts)
+        return applied
 
     def solve(self, starts, sigma, dw, dc, rhs):
         out = self.ev.kkt_solve(starts, sigma, dw, dc, rhs)
@@ -59,18 +80,34 @@ def _bounds(v, size, fill):
     return np.full(size, fill) if v is None else np.array(v, dtype=np.float64).reshape(size)
 
 
-def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_iter=500, mu_init=0.1, progress=None):
+HESSIAN_APPROXIMATIONS = ("exact", "limited-memory")
+
+
+def check_hessian_approximation(value):
+    if value not in HESSIAN_APPROXIMATIONS:
+        raise ValueError("hessian_approximation must be 'exact' or 'limited-memory', not %r" % (value,))
+    return value == "limited-memory"
+
+
+def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_iter=500, mu_init=0.1, progress=None,
+                 hessian_approximation="exact"):
     """Solve min f(x) s.t. cl <= g(x) <= cu, lb <= x <= ub from every row of ``X0`` (B, n) in lock step.
 
     ``ev``: batched evaluator (``BatchedOracles`` or anything with ``eval(X, LAM, SIGMA, want) -> {name: (B, len)}``,
     ``jacobianstructure()``, ``n``, ``m``); ``kkt``: KKT backend (``DeviceKKT(ev)`` or one with the same
     ``setup`` / ``load`` / ``solve``).  Bounds beyond 1e19 in magnitude are absent, as for IPOPT.
+    ``hessian_approximation``: "exact" or "limited-memory" (damped BFGS per start, see the module docstring); the
+    latter needs a backend built for it (``quasi_newton = True``, with ``update(starts, S, Y)``).
 
     Returns per start: ``x``, ``g``, ``f``, ``lam`` (constraint multipliers, IPOPT's mult_g), ``zL``, ``zU`` (bound
     multipliers), ``status`` (0 solved, -1 iteration limit, 3 step too small, -3 KKT system could not be regularised,
     -13 invalid number) and ``iterations``; plus ``timings``: per outer iteration the wall seconds spent in evaluations
     (``eval_s``), in the KKT backend (``kkt_s``) and in total (``total_s``).  ``progress(it, timing, n_active)``, when
     given, is called after every outer iteration (long batches run for minutes)."""
+    qn = check_hessian_approximation(hessian_approximation)
+    if bool(getattr(kkt, "quasi_newton", False)) != qn:
+        raise ValueError("hessian_approximation=%r needs a KKT backend with quasi_newton=%s"
+                         % (hessian_approximation, qn))
     X0 = np.array(X0, dtype=np.float64, ndmin=2)
     B, n = X0.shape
     m = int(ev.m)
@@ -148,6 +185,7 @@ def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_
         iters = np.zeros(B, dtype=np.int64)
         active = np.ones(B, dtype=bool)
         f = np.zeros(B)
+        qn_from = None                 # (accepted, x, grad f, J) of the previous iteration, for the BFGS update
         timings = []
         for it in range(max_iter + 1):
             t0 = time.perf_counter()
@@ -180,6 +218,16 @@ def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_
             if not active.any():
                 timings.append({"eval_s": t_eval, "kkt_s": 0.0, "total_s": time.perf_counter() - t0})
                 break
+            t_qn = 0.0
+            if qn_from is not None:        # damped BFGS with the previous iteration's step, at the new lam
+                t1 = time.perf_counter()
+                acc_prev, X_old, grad_old, J_old = qn_from
+                idx = np.flatnonzero(acc_prev & active)
+                if idx.size:
+                    Yn = res["grad"][idx] + np.matmul(lam[idx, None, :], J[idx])[:, 0, :]
+                    Yo = grad_old[idx] + np.matmul(lam[idx, None, :], J_old[idx])[:, 0, :]
+                    kkt.update(idx, X[idx] - X_old[idx], Yn - Yo)
+                t_qn = time.perf_counter() - t1
             while True:                # monotone barrier update
                 upd = active & (mu > tol / 10.0) & (err(mu) <= 10.0 * mu)
                 if not upd.any():
@@ -212,7 +260,7 @@ def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_
                 dw[rej] = np.where(d == 0.0, np.maximum(d0 / 3.0, 1e-4),
                                    d * np.where((d0 == 0.0) & (attempt < 3), 100.0, 8.0))
                 pend[rej[dw[rej] > 1e40]] = False
-            t_kkt = time.perf_counter() - t1
+            t_kkt = time.perf_counter() - t1 + t_qn
             solved = active & np.isfinite(sol).all(axis=1)
             failed = active & ~solved
             status[failed], iters[failed], active[failed] = -3, it, False
@@ -265,6 +313,8 @@ def lockstep_ipm(ev, kkt, X0, lb=None, ub=None, cl=None, cu=None, tol=1e-8, max_
             stop = accepted & (stalled >= 30)  # the l1 merit line search has no filter / SOC
             status[stop], iters[stop], active[stop] = 3, it, False
             acc = accepted & ~stop
+            if qn:
+                qn_from = (acc, X, res["grad"], J)
             Z = np.where(acc[:, None], Zacc, Z)
             X = Z[:, :n].copy()
             f = np.where(acc, facc, f)

@@ -108,16 +108,42 @@ class BatchedOracles:
         return self.dev._L.dnlp_batch_instr_kernel(self.dev.h, int(instr)).decode()
 
     # ---- batched KKT systems (dnlp_b200/lockstep_ipm.py; include/dnlp_b200.h dnlp_batch_kkt_*) ---------------
-    def kkt_setup(self, slack_rows):
+    def kkt_setup(self, slack_rows, quasi_newton=False):
         """Scatter maps of K = [[W + diag(Sigma) + dw I, A'], [A, -dc I]], A = [J, -P], for the slack rows
-        ``slack_rows`` (the inequality rows, in slack order), and B dense systems in HBM."""
+        ``slack_rows`` (the inequality rows, in slack order), and B dense systems in HBM.  W is the HESS output, or
+        with ``quasi_newton`` one damped-BFGS matrix per start kept in HBM (set to I here, see ``qn_update``)."""
         sr = np.ascontiguousarray(slack_rows, dtype=np.int32)
-        pats = [np.ascontiguousarray(a, dtype=np.int32) for a in
-                (self.tape.jac_rows, self.tape.jac_cols, self.tape.hess_rows, self.tape.hess_cols)]
-        self.dev.check(self.dev._L.dnlp_batch_kkt_setup(self.dev.h, int(sr.size), sr.ctypes.data_as(_cabi.c_i32p),
-                                                        *[a.ctypes.data_as(_cabi.c_i32p) for a in pats]))
+        names = ("jac_rows", "jac_cols") if quasi_newton else ("jac_rows", "jac_cols", "hess_rows", "hess_cols")
+        pats = [np.ascontiguousarray(getattr(self.tape, a), dtype=np.int32) for a in names]
+        setup = self.dev._L.dnlp_batch_kkt_setup_qn if quasi_newton else self.dev._L.dnlp_batch_kkt_setup
+        self.dev.check(setup(self.dev.h, int(sr.size), sr.ctypes.data_as(_cabi.c_i32p),
+                             *[a.ctypes.data_as(_cabi.c_i32p) for a in pats]))
         self.kkt_N = self.n + int(sr.size)
         self.kkt_ms = 0.0
+        self.qn_ms = 0.0
+
+    def qn_update(self, starts, S, Y):
+        """Damped BFGS update of the quasi-Newton matrices of the start ids ``starts`` with the steps ``S`` and the
+        gradient changes ``Y`` (count, n) (the update of the test-suite's stand-in, include/dnlp_b200.h).  Returns
+        ``applied`` (count,) bool: False where s'Ws > 0 fails and W is left as it was.  ``qn_ms`` keeps the
+        CUDA-event time of the call's kernels."""
+        st = np.ascontiguousarray(starts, dtype=np.int32).reshape(-1)
+        cnt = st.size
+        S = np.ascontiguousarray(S, dtype=np.float64).reshape(cnt, self.n)
+        Y = np.ascontiguousarray(Y, dtype=np.float64).reshape(cnt, self.n)
+        applied = np.zeros(cnt, dtype=np.int32)
+        ms = C.c_float(0)
+        self.dev.check(self.dev._L.dnlp_batch_qn_update(self.dev.h, int(cnt), st.ctypes.data_as(_cabi.c_i32p),
+                                                        _ptr(S), _ptr(Y), applied.ctypes.data_as(_cabi.c_i32p),
+                                                        C.byref(ms)))
+        self.qn_ms = float(ms.value)
+        return applied.astype(bool)
+
+    def qn_matrix(self, start):
+        """The quasi-Newton matrix of start ``start``, (n, n)."""
+        out = np.empty((self.n, self.n))
+        self.dev.check(self.dev._L.dnlp_batch_qn_matrix(self.dev.h, int(start), _ptr(out)))
+        return out
 
     def kkt_solve(self, starts, sigma, dw, dc, rhs):
         """Assemble, factor (LDL', no pivoting) and solve the systems of the start ids ``starts`` from the JAC and

@@ -222,6 +222,22 @@ int dnlp_batch_kkt_solve(dnlp_batch *b, int32_t count, const int32_t *starts, co
                          float *elapsed_ms);
 int dnlp_batch_kkt_matrix(dnlp_batch *b, int32_t start, double *out);
 
+/* Quasi-Newton mode (hessian_approximation = "limited-memory" of the lock-step driver): W_b is a dense damped-BFGS
+ * matrix per start kept in HBM instead of the HESS output, its lower triangle packed batch fastest (entry (i, j <= i)
+ * of start b at (i(i+1)/2 + j) * B + b).  dnlp_batch_kkt_setup_qn builds the scatter map from the JAC pattern, the
+ * slack -1 entries and the packed W (no HESS source), allocates the K and W workspaces and sets every W_b = I; it
+ * fails with a message naming B*(N+m)^2*8 and B*n(n+1)/2*8 bytes when they do not fit, or when n(n+1)/2 plus the
+ * Jacobian entries exceed the int32 range.  It and dnlp_batch_kkt_setup replace each other's state.
+ * dnlp_batch_kkt_solve and dnlp_batch_kkt_matrix work in both modes.
+ * dnlp_batch_qn_update applies the damped BFGS update of the test-suite's stand-in to `count` distinct start ids:
+ * S and Y are start-major (S[c*n + i]); applied[c] = 0 when s'Ws > 0 fails (NaN included) and W_b is left unchanged.
+ * *elapsed_ms: CUDA-event time of the update's kernels.  dnlp_batch_qn_matrix copies W_b as a full n x n matrix. */
+int dnlp_batch_kkt_setup_qn(dnlp_batch *b, int64_t ns, const int32_t *slack_rows, const int32_t *jac_rows,
+                            const int32_t *jac_cols);
+int dnlp_batch_qn_update(dnlp_batch *b, int32_t count, const int32_t *starts, const double *S, const double *Y,
+                         int32_t *applied, float *elapsed_ms);
+int dnlp_batch_qn_matrix(dnlp_batch *b, int32_t start, double *out);
+
 /* ---- row-sharded evaluation across the GPUs of one node (BASELINE config 3; SURVEY.md 8e) ----
  * One process per GPU.  The reference has no counterpart (it is single-process NumPy); the surface
  * mirrors the callbacks above, evaluated collectively: every rank runs the local tape of its rows,
